@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                   # this repo's CUDA path, BASELINE configs[2]
     python bench.py --config c2|c3|c4 ...                            # the other single-GPU configs of BASELINE.json
     python bench.py --impl reference --gpus N --steps K --warmup W  # the reference algorithm on the host CPU
+    python bench.py ... --dump-outputs DIR                           # also save the last timed step's results
 
 Workloads (BASELINE.json `configs`):
   c3 (default)  large-v3, beam 5, batch 64 per GPU, bf16, kv-cache; one "step" = one pass of the whole hot path over
@@ -69,7 +70,12 @@ def parse():
                     help="after the timed region, run one extra plain-launch step per kernel class with per-launch "
                          "CUDA events and report each class's total device time (diagnostic, not part of `value`)")
     ap.add_argument("--breakdown-ids", default="1,2,3,4,5,6,7,8", help="kernel classes for --breakdown")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64; token rows padded with -1), "
+                         "so that two builds can be compared output for output on the same seeded inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     model, batch, beam, dtype, mode = PRESETS[args.config]
     args.model = args.model or model
     args.batch = args.batch or batch
@@ -171,6 +177,27 @@ def algorithmic_numbers(dims, B, G, L_avg):
     out["decode_step_bytes"] = (out["decoder_weight_bytes_per_step"] + out["cross_kv_bytes_per_step"] +
                                 out["self_kv_bytes_per_step_avg"] + out["kv_append_and_logits_bytes_per_step"])
     return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def padded_rows(rows):
+    """Token lists as one float64 matrix, short rows padded with -1 (token ids are exact in float64)."""
+    out = np.full((len(rows), max((len(r) for r in rows), default=0)), -1.0)
+    for i, r in enumerate(rows):
+        out[i, :len(r)] = r
+    return out
+
+
+def dump_outputs(directory, arrays):
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit; use a smaller workload")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def host_threads() -> int:
@@ -413,9 +440,8 @@ def main():
     def hot_path(audio):
         mel = wb.log_mel_spectrogram(audio, dims["n_mels"], per_waveform_max=True)   # each segment = its own file
         res = model.decode(mel, options)
-        toks, lps, nss = parallel.gather_results([r.tokens for r in res], [r.avg_logprob for r in res],
-                                                 [r.no_speech_prob for r in res], dev)
-        return toks
+        return parallel.gather_results([r.tokens for r in res], [r.avg_logprob for r in res],
+                                       [r.no_speech_prob for r in res], dev)
 
     def step_resident():
         return hot_path(audio_dev)
@@ -425,7 +451,7 @@ def main():
 
     for _ in range(max(3, args.warmup)):
         out = step_resident()
-    n_tokens = [len(t) for t in out]
+    n_tokens = [len(t) for t in out[0]]
 
     sampler = ClockSampler(local)
     if rank == 0:
@@ -438,6 +464,9 @@ def main():
     model.timing = None
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        toks, lps, nss = out
+        dump_outputs(args.dump_outputs, {"tokens": padded_rows(toks), "avg_logprob": lps, "no_speech_prob": nss})
 
     # roofline of the dominant kernel (decoder-step cross-attention): one more step with every launch of
     # that kernel bracketed by CUDA events on its stream.  This pass runs the decode loop as plain launches
@@ -595,6 +624,12 @@ def bench_transcribe(args, model, tok, dims, dev, rank, world, local, timed, lib
     model.timing = None
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        segs = res["segments"]
+        dump_outputs(args.dump_outputs, {"tokens": padded_rows([s["tokens"] for s in segs]),
+                                         **{k: [s[k] for s in segs] for k in ("seek", "start", "end", "temperature",
+                                                                             "avg_logprob", "compression_ratio",
+                                                                             "no_speech_prob")}})
     e2e_steps = max(1, min(args.steps, 2))
     ms_e2e, _ = timed(lambda: run(audio_host.to(dev, non_blocking=True)), e2e_steps)
     # lock-step over 16 files of the same total duration

@@ -17,6 +17,7 @@ Fixtures:
   model_<name>.npz/.json   encoder features (sub-sampled), prefill logits probes, and decode()
                            results (tokens, avg_logprob, no_speech_prob) for several DecodingOptions
   decode_extra_<name>.json decode() with task="translate", other language tokens, language=None and task="lang_id"
+  checkpoints_reference.json  download URL and alignment-head dump per official model name
   state_dict_keys.json     names and shapes of the reference Whisper.state_dict() per architecture
   transcribe_<name>.json   whisper.transcribe() runs (transcribe.py:38-514) recorded as: every model.decode() call
                            the reference made (prompt, temperature, beam / best_of, a fingerprint of the window) with
@@ -366,10 +367,24 @@ def gen_state_dict_keys():
     print("state dict keys:", {k: len(v) for k, v in out.items()})
 
 
+def gen_checkpoints():
+    """Per official model name: the reference's download URL (its last two components are the cached file's SHA-256
+    and name, __init__.py:17-32) and its alignment-head dump (:36-51)."""
+    out = {name: {"url": url, "alignment_heads": whisper._ALIGNMENT_HEADS[name].decode()
+                  if name in whisper._ALIGNMENT_HEADS else None}
+           for name, url in whisper._MODELS.items()}
+    with open(os.path.join(GOLD, "checkpoints_reference.json"), "w") as f:
+        json.dump(out, f, indent=1)
+    print("checkpoints:", len(out))
+
+
 def main():
     torch.set_num_threads(os.cpu_count() or 1)
     if sys.argv[1:] == ["test-peak"]:        # only the round-2 fixture (the others are unchanged since round 1)
         gen_model("test-peak", seed=21, audio_kind="speechlike", full_length=False, regime="peaked", cases=PEAKED_CASES)
+        return
+    if sys.argv[1:] == ["checkpoints"]:
+        gen_checkpoints()
         return
     gen_static()
     gen_timing()
@@ -382,6 +397,7 @@ def main():
     gen_transcribe("test-multi", seed=12, regime="diverse")
     gen_state_dict_keys()
     gen_decode_extra("test-multi", seed=12, audio_kind="noise", regime="diverse")
+    gen_checkpoints()
     print("golden fixtures written to", GOLD)
 
 

@@ -2,7 +2,6 @@
 suppress lists, hypothesis finalisation / ranking, window splitting, padding, id tables."""
 import json
 import os
-import sys
 from types import SimpleNamespace
 
 import numpy as np
@@ -560,15 +559,13 @@ def test_official_checkpoint_table_and_sha256_gate(tmp_path):
             d = wb.dims_dict(name)
             mask = np.frombuffer(gzip.decompress(base64.b85decode(e["alignment_heads"].encode())), dtype=bool)
             assert mask.size == d["n_text_layer"] * d["n_text_head"] and mask.any()
-    if os.path.isdir("/root/reference/whisper"):      # in the build container: the table IS the reference's
-        sys.path.insert(0, "/root/reference")
-        try:
-            import whisper as ref
-            for name, url in ref._MODELS.items():
-                assert table[name]["file"] == os.path.basename(url) and table[name]["sha256"] == url.split("/")[-2]
-                assert (table[name]["alignment_heads"] or "").encode() == ref._ALIGNMENT_HEADS.get(name, b"")
-        finally:
-            sys.path.remove("/root/reference")
+    # the table IS the reference's (its _MODELS / _ALIGNMENT_HEADS, stored by oracle/make_golden.py: gen_checkpoints)
+    with open(os.path.join(GOLD, "checkpoints_reference.json")) as f:
+        ref = json.load(f)
+    assert set(ref) == set(table)
+    for name, e in ref.items():
+        assert table[name]["file"] == os.path.basename(e["url"]) and table[name]["sha256"] == e["url"].split("/")[-2]
+        assert table[name]["alignment_heads"] == e["alignment_heads"]
     # a file under the official name with other contents is refused before anything touches the GPU
     (tmp_path / "tiny.en.pt").write_bytes(b"not the official checkpoint")
     with pytest.raises(RuntimeError, match="SHA256"):
